@@ -7,7 +7,7 @@ into baseline/_ref/src, sha256 recorded) against two tiny stand-ins kept in base
 over POSIX shm (mpi.h / egmpi.c / mpirun) and a header-only opencv2/opencv.hpp that synthesises CIFAR-shaped images.
 `pip install /root/reference` was tried first, as prescribed, and fails (no setup.py / pyproject) -- see README.md.
 
-    python baseline/build_ref.py [--ref /root/reference] [--only cifar_event,...]
+    python baseline/build_ref.py --ref <reference checkout> [--only cifar_event,...]
 """
 from __future__ import annotations
 import argparse, hashlib, json, os, shutil, subprocess, sys, time
@@ -24,7 +24,7 @@ PROGRAMS = {  # binary name -> source relative to the reference root
 
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("--ref", default="/root/reference")
+    ap.add_argument("--ref", required=True, help="checkout of the reference programs")
     ap.add_argument("--only", default="")
     ap.add_argument("--out", default=os.path.join(HERE, "_ref"))
     a = ap.parse_args()

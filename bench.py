@@ -15,6 +15,8 @@ One JSON line on rank 0.  `value` is timed on the device (CUDA events) over K wh
 (forward, backward, fused exchange+average+SGD) with inputs already resident; `e2e` repeats the
 measurement through the public Trainer API with, every step, the H2D copy of that step's uint8
 batch from pinned host memory, GPU decode/augmentation, and a D2H read of the loss.
+`--dump-outputs DIR` writes what the last device-timed step computed as DIR/<name>.npy; the inputs are seeded, so
+two builds run with the same arguments can be compared output for output.
 The headline runs at the reference's precision (fp32, TF32 off) with the Trainer's DEFAULT execution
 switches (on a GPU: NHWC + fused BN kernels, whole-step CUDA graph, overlapped pushes for N >= 2) -- the
 same configuration `python -m eventgrad_b200.cli.cifar_event` uses; bf16 / tf32 rows ride along under
@@ -67,7 +69,34 @@ def parse():
     p.add_argument("--no-e2e", action="store_true")
     p.add_argument("--out", default="")
     p.add_argument("--profile", default="", help="write a torch.profiler kernel table of a few e2e steps here")
+    p.add_argument("--dump-outputs", default="", metavar="DIR",
+                   help="after the timed steps, write what the last one computed (loss, a fixed seeded sample of the "
+                        "updated parameters, the BatchNorm running statistics) as DIR/<name>.npy in float32")
     return p.parse_args()
+
+
+DUMP_PARAM_SAMPLE = 1 << 22          # parameters written by --dump-outputs over all ranks (16 MB of float32)
+
+
+def dump_outputs(tr, out_dir, rank, world):
+    """Write what the last step handed its caller as float32 .npy files: the loss it returned, the updated
+    parameters (a fixed, seeded sample of their concatenation in named_parameters() order) and the BatchNorm
+    running statistics.  The inputs are seeded, so two builds run with the same arguments compare file by file."""
+    import numpy as np
+    import torch
+    params = torch.cat([p.detach().reshape(-1) for p in tr.model.parameters()]).float().cpu()
+    k = DUMP_PARAM_SAMPLE // world
+    if params.numel() > k:
+        idx = torch.randperm(params.numel(), generator=torch.Generator().manual_seed(0))[:k].sort().values
+        params = params[idx]
+    stats = [b.detach().reshape(-1).float() for b in tr.model.buffers() if b.is_floating_point()]
+    arrays = {"loss": tr.last_loss.detach().float().reshape(1).cpu(), "params_sample": params,
+              "bn_running_stats": torch.cat(stats).cpu() if stats else torch.zeros(0)}
+    sfx = f"_rank{rank}" if world > 1 else ""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + sfx + ".npy"), a.numpy().astype(np.float32))
+    return sorted(name + sfx + ".npy" for name in arrays)
 
 
 def reference_arm(args):
@@ -78,9 +107,10 @@ def reference_arm(args):
     return ref_arm.run(args)
 
 
-def measure(args, env, dtype, want_e2e, src, sample_clocks):
+def measure(args, env, dtype, want_e2e, src, sample_clocks, dump_dir=""):
     """One Trainer at `dtype`: device-timed K steps (+ optionally the end-to-end loop).  Returns a dict.
-    `fp32_cudnn` = fp32 with the tensor-core convolutions switched off (cuDNN's SIMT fp32 kernels, NCHW)."""
+    `fp32_cudnn` = fp32 with the tensor-core convolutions switched off (cuDNN's SIMT fp32 kernels, NCHW).
+    With `dump_dir`, what the last device-timed step computed is written there before anything else runs."""
     conv_tc = {"auto": None, "on": True, "off": False}[args.conv_tc]
     if dtype == "fp32_cudnn":
         dtype, conv_tc = "fp32", False
@@ -141,6 +171,8 @@ def measure(args, env, dtype, want_e2e, src, sample_clocks):
            "loss": float(tr.last_loss), "clocks": clocks, "gpu_launches": int(own_launches),
            "own_kernels_per_step": dict(tr.own_launches_per_step), "cfg": cfg, "gb": gb, "per_rank": per_rank,
            "table": table, "algo": algo, "backend": backend}
+    if dump_dir:
+        res["dumped"] = dump_outputs(tr, dump_dir, env.rank, N)
 
     # ---------------- end to end through the public API: H2D every step + D2H loss every step ----
     if want_e2e:
@@ -249,7 +281,7 @@ def main():
     gb = args.global_batch if args.scaling == "strong" else args.global_batch * N
     n_train = max(max(1, gb // N) * N * 8, 4096)
     src = synthetic_source("cifar10", n_train).pin()
-    r = measure(args, env, args.dtype, not args.no_e2e, src, True)
+    r = measure(args, env, args.dtype, not args.no_e2e, src, True, args.dump_outputs)
     others = {}
     for dt in [d for d in args.also.split(",") if d and d != args.dtype]:
         if dt == "fp32_cudnn" and (args.dtype != "fp32" or not r["cfg"].conv_tc):
@@ -300,6 +332,9 @@ def main():
         out["e2e"] = r["e2e"]
     if others:
         out["other_dtypes"] = others
+    if "dumped" in r:
+        out["outputs_dumped"] = {"dir": args.dump_outputs, "files": r["dumped"],
+                                 "of": "the last device-timed step of the headline dtype"}
     if env.rank == 0:
         line = json.dumps(out)
         print(line, flush=True)

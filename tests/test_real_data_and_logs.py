@@ -84,9 +84,22 @@ def test_reference_log_formats(tmp_path):
             assert open(d / "train2.txt").read() == "7, 0.123457\n"                     # iostream default = %g
 
 
+def _check_reference_line(d):
+    assert d["impl"] == "reference"
+    assert d["value"] > 0 and d["unit"] == "images/s" and d["dtype"] == "fp32" and d["steps"] == 1
+    assert d["config"]["identical_to_reference"] is True and d["gpu_launches"] == 0
+    assert d["e2e"]["value"] == d["value"]
+
+
 def test_bench_reference_arm_contract():
     """`bench.py --impl reference` either times the unmodified reference (baseline/_ref built) and prints the bench
-    schema with impl=reference, or says why it cannot -- always one JSON line, exit 0, none of our package loaded."""
+    schema with impl=reference, or says why it cannot -- always one JSON line, exit 0, none of our package loaded.
+    tests/golden holds the line the reference's cifar_event printed for these arguments (CPU, 8 cores): it must meet
+    the same schema, and a live run must have been built from the same source and start from the same loss (the
+    program seeds its weights, sampler and transforms)."""
+    with open(os.path.join(ROOT, "tests", "golden", "reference_arm_cifar_event.json")) as f:
+        golden = json.load(f)
+    _check_reference_line(golden)
     env = dict(os.environ, EGREF_BUDGET_S="240")
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "1",
                         "--steps", "1", "--warmup", "0"], capture_output=True, text=True, timeout=600, env=env)
@@ -96,6 +109,7 @@ def test_bench_reference_arm_contract():
     if "unavailable" in d:
         assert isinstance(d["unavailable"], str) and d["unavailable"]
     else:
-        assert d["value"] > 0 and d["unit"] == "images/s" and d["dtype"] == "fp32" and d["steps"] == 1
-        assert d["config"]["identical_to_reference"] is True and d["gpu_launches"] == 0
-        assert d["e2e"]["value"] == d["value"]
+        _check_reference_line(d)
+        for k in ("source_sha256", "program", "model", "global_batch"):
+            assert d["config"][k] == golden["config"][k], k
+        assert np.allclose(d["loss_first_last"], golden["loss_first_last"], rtol=1e-3, atol=0)
