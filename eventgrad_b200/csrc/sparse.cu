@@ -264,7 +264,7 @@ __global__ void __launch_bounds__(EG_THREADS, 4) sparse_cand_kernel(const Sparse
     const uint32_t* cand = p.cand + (size_t)p.tab.t_tile_start[i] * EG_TILE;
     const unsigned n = __ldcg(p.cand_cnt + i);
     unsigned remain = p.sel_remain[i];
-    // digit 2: bits [20:10]
+    // digit 2: bits [19:9]
     __syncthreads();
     for (int bkt = tid; bkt < SP_BINS; bkt += EG_THREADS) sh[bkt] = 0u;
     __syncthreads();
@@ -283,7 +283,7 @@ __global__ void __launch_bounds__(EG_THREADS, 4) sparse_cand_kernel(const Sparse
     unsigned d2, above;
     block_pick(sh, SP_BINS, remain, &d2, &above);
     remain -= above;
-    // digit 3: bits [9:0] among the candidates that match digit 2
+    // digit 3: bits [8:0] among the candidates that match digit 2
     __syncthreads();
     for (int bkt = tid; bkt < (1 << SP_SH2); bkt += EG_THREADS) sh[bkt] = 0u;
     __syncthreads();
